@@ -2,6 +2,7 @@
 bf16, sequence length 4096, synthetic packed tokens, random-init weights — BASELINE.json's metric and config.
 
     python bench.py --gpus N --steps K --warmup W                 # this framework
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # ... and write the last timed step's results
     python bench.py --impl reference --gpus N --steps K --warmup W   # the unmodified reference from baseline/_ref
     (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py ...)
 
@@ -25,6 +26,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
@@ -174,7 +176,8 @@ def run(args) -> dict:
         raise SystemExit(f"--config {args.config} needs a multiple of {MODEL['tp']} GPUs (tensor parallel degree)")
     dp = world // MODEL["tp"]
     mbs, T, V = args.mbs, MODEL["sequence_length"], MODEL["vocab_size"]
-    tmp = Path(os.environ.get("MB200_BENCH_TMP", "/tmp/mb200_bench"))
+    # configs and the warm-start checkpoint: outside the tree, one directory per user shared by the ranks of a run
+    tmp = Path(os.environ.get("MB200_BENCH_TMP") or Path(tempfile.gettempdir()) / f"mb200_bench_{os.getuid()}")
     cfg_path = write_config(args.impl, mbs, world, args.steps * 2 + args.warmup * 2 + 4, tmp)
 
     if args.impl == "reference":
@@ -199,6 +202,7 @@ def run(args) -> dict:
         from modalities_b200.ops import functional as OF
 
         OF.set_fp8(True)
+    torch.manual_seed(0)  # the same random-init weights in every run (--dump-outputs compares runs output for output)
     main = Main(cfg_path, experiments_root_path=tmp / "experiments", experiment_id=f"bench_{args.impl}")
     components = main.build_components(components_model_type=model_type)
     model = components.app_state.model_parts[0]
@@ -244,6 +248,7 @@ def run(args) -> dict:
     pool = [host_batch() for _ in range(4)]
     h2d_bytes = sum(t.numel() * t.element_size() for t in pool[0])
     counter = _LaunchCounter(args.impl)
+    last_step = {}  # what the latest training step returned: loss and gradient norm (device tensors)
 
     def step(i: int, from_host: bool, dev_batch=None):
         if from_host:
@@ -257,6 +262,7 @@ def run(args) -> dict:
             batch = DatasetBatch(samples={"input_ids": dev_batch[0]}, targets={"target_ids": dev_batch[1]})
         _, _, loss, grad_norm = trainer._train_batch(batch=batch, model_parts=[model], optimizer=optimizer, scheduler=scheduler,
                                                      loss_fun=components.loss_fn, micro_batch_id=i)  # fmt: skip
+        last_step.update(loss=loss, grad_norm=grad_norm)
         if from_host:
             return float(loss.detach().float().item())  # device→host read of the step result
         return loss
@@ -316,6 +322,8 @@ def run(args) -> dict:
         busy_ms = rt.comm_busy_ms() / (args.steps + args.warmup)
         rt.comm_meter = False
     ms_e2e, wall_e2e, clocks_e2e, _, loss_e2e = timed(from_host=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), last_step, model)
 
     if args.profile:
         from torch.profiler import ProfilerActivity, profile
@@ -390,6 +398,26 @@ def run(args) -> dict:
     return result if rank == 0 else {}
 
 
+def dump_outputs(out_dir: Path, last_step: dict, model, per_param: int = 4096) -> None:
+    """The results of the last timed step as float32 .npy files: ``loss`` and ``grad_norm`` (what the training step returns)
+    and ``params_sample``, the updated parameters of this rank at ``per_param`` seeded positions of every parameter in
+    ``named_parameters`` order (a fixed sample: 2.7B parameters would not fit the 64 MB the dump may take)."""
+    import numpy as np
+    import torch
+
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name in ("loss", "grad_norm"):
+        np.save(out_dir / f"{name}.npy", last_step[name].detach().float().reshape(1).cpu().numpy())
+    gen = torch.Generator().manual_seed(0)
+    samples = []
+    with torch.no_grad():
+        for _, p in model.named_parameters():
+            flat = (p.to_local() if hasattr(p, "to_local") else p).detach().reshape(-1)
+            idx = torch.randint(0, flat.numel(), (min(per_param, flat.numel()),), generator=gen)
+            samples.append(flat[idx.to(flat.device)].float().cpu())
+    np.save(out_dir / "params_sample.npy", torch.cat(samples).numpy())
+
+
 def _warmstart_roundtrip(impl: str, components, folder: Path, rank: int):
     """Instruction-tuning runs start from pretrained weights: write this run's (sharded, DTensor) model state dict with
     torch.distributed.checkpoint and load it back into the live model through each package's own state-dict hooks
@@ -458,7 +486,12 @@ def main():
                          "(BASELINE config 4); everything else as in the bf16 run. Own arm only.")
     ap.add_argument("--profile", type=str, default=None,
                     help="after the timed passes, run 2 more steps under torch.profiler on rank 0 and write the per-kernel table here")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="after the timed passes, write the loss, gradient norm and a fixed sample of the updated parameters of the "
+                         "last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -1,5 +1,6 @@
 import os
 import sys
+import tempfile
 from pathlib import Path
 
 import pytest
@@ -8,11 +9,23 @@ REPO = Path(__file__).resolve().parents[1]
 if str(REPO) not in sys.path:
     sys.path.insert(0, str(REPO))
 
+# transformers copies the code of a trust_remote_code model into HF_MODULES_CACHE (by default under HF_HOME, which need not
+# be writable by the user running the tests); the tests export and reload such models, so the copies go to a temporary
+# directory of the session — set before anything imports transformers, and inherited by the tests' subprocesses
+_HF_MODULES = tempfile.TemporaryDirectory(prefix="mb200_hf_modules_")
+os.environ["HF_MODULES_CACHE"] = _HF_MODULES.name
+
 DATA = REPO / "data"
+# what the reference implementation computes for the differential tests (scripts/reference_goldens.py writes it)
+REFERENCE_GOLDEN = REPO / "tests" / "golden" / "reference"
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: test needs a CUDA device (run on the B200 box: pytest -m gpu)")
+
+
+def pytest_unconfigure(config):
+    _HF_MODULES.cleanup()
 
 
 def pytest_collection_modifyitems(config, items):
@@ -55,6 +68,13 @@ def dist_env_single(free_port, monkeypatch):
     dist.init_process_group("gloo")
     yield
     dist.destroy_process_group()
+
+
+def reference_golden(name: str):
+    import gzip
+    import json
+
+    return json.loads(gzip.decompress((REFERENCE_GOLDEN / f"{name}.json.gz").read_bytes()))
 
 
 def run_arms(make_cmd, arms=("ref", "ours"), cwd=None, env=None, timeout=600):

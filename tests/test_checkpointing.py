@@ -176,25 +176,28 @@ def test_fsdp1_full_state_files_and_deletion(tmp_path, dist_env_single):
 
 def test_checkpoint_written_through_the_reference_classes_loads_here(tmp_path):
     """The opposite direction of the cross-load in test_engine.py: the REFERENCE's AppState + torch AdamW + OneCycleLR
-    (baseline/_ref) train three steps and ``dcp.save`` a checkpoint; this framework's AppState restores it — into plain torch
-    objects and into the sharded runtime + FusedAdamW — with the same weights, Adam moments and step, learning rate and
-    scheduler position the reference reports."""
+    trained a tiny GPT2LLM three steps and wrote a checkpoint with ``dcp.save`` (tests/golden/reference/tiny_checkpoint.*);
+    this framework's AppState restores it — into plain torch objects and into the sharded runtime + FusedAdamW — with the
+    same weights, Adam moments and step, learning rate and scheduler position the reference reports."""
     import json
     import subprocess
     import sys
+    import tarfile
     from pathlib import Path
 
+    from conftest import REFERENCE_GOLDEN, reference_golden
+
     repo = Path(__file__).resolve().parents[1]
-    if not (repo / "baseline" / "_ref" / "modalities").is_dir():
-        pytest.skip("the reference is not installed under baseline/_ref")
-    ckpt = tmp_path / "ref_ckpt"
+    with tarfile.open(REFERENCE_GOLDEN / "tiny_checkpoint.tar.gz") as tar:
+        tar.extractall(tmp_path, filter="data")
+    ckpt = tmp_path / "tiny_checkpoint"
 
     def run(*args):
         r = subprocess.run([sys.executable, "tests/workers/reference_checkpoint_load.py", *args], cwd=repo, capture_output=True, text=True, timeout=600)
         assert r.returncode == 0, r.stderr[-3000:]
         return json.loads(r.stdout.strip().splitlines()[-1])
 
-    written = run("ref", str(ckpt), "save")
-    assert written["adam_steps"] == [3.0] and written["n_state"] == 21
-    assert run("ours", str(ckpt)) == written
-    assert run("ours_sharded", str(ckpt)) == written
+    written = reference_golden("tiny_checkpoint")
+    assert written["adam_steps"] == [3.0] and written["n_state"] == 19
+    assert run("ours", str(ckpt), "tiny") == written
+    assert run("ours_sharded", str(ckpt), "tiny") == written

@@ -113,15 +113,13 @@ def test_unknown_keys_missing_components_and_cycles():
 
 
 def test_registry_matches_reference_catalogue():
-    import re
-
     from modalities_b200.registry.components import COMPONENTS
 
+    from conftest import reference_golden
+
     mine = {(e.component_key, e.variant_key) for e in COMPONENTS}
-    ref_file = Path("/root/reference/src/modalities/registry/components.py")
-    if ref_file.exists():
-        ref = set(re.findall(r'ComponentEntity\(\s*"([a-z_0-9]+)",\s*"([a-z_0-9]+)"', ref_file.read_text()))
-        assert ref <= mine, sorted(ref - mine)
+    ref = {tuple(e) for e in reference_golden("components")}  # the ComponentEntity entries of the reference's registry
+    assert len(ref) >= 90 and ref <= mine, sorted(ref - mine)
     assert len(mine) >= 94
 
 
@@ -170,22 +168,16 @@ def test_custom_model_example_trains_through_main(tmp_path):
 def test_component_nodes_of_the_reference_yaml_files_fit_our_schemas():
     """Schema parity, checked mechanically: every ``{component_key, variant_key, config}`` node in the reference's shipped
     training / data-preparation / tutorial / test YAML files must name a registered component and use only config keys that
-    our pydantic schema of that component knows (deprecated aliases included). Needs the reference checkout (skipped
-    otherwise); its unit-test fixtures with made-up components (COMP_X …, dataset/test) are not real configs."""
-    import glob
-    from pathlib import Path
-
-    import yaml
+    our pydantic schema of that component knows (deprecated aliases included). The nodes are those recorded from the
+    reference's files in tests/golden/reference/yaml_nodes.json.gz; its unit-test fixtures with made-up components (COMP_X …,
+    dataset/test) are not real configs."""
+    from conftest import reference_golden
 
     from modalities_b200.registry.components import COMPONENTS
 
-    ref = Path("/root/reference")
-    if not ref.exists():
-        pytest.skip("reference checkout not available")
+    golden = reference_golden("yaml_nodes")
     entities = {(c.component_key, c.variant_key): c for c in COMPONENTS}
-    files = [f for pattern in ("config_files/**/*.yaml", "tutorials/**/*.yaml", "tests/**/*.yaml")
-             for f in glob.glob(str(ref / pattern), recursive=True)]  # fmt: skip
-    assert len(files) > 50
+    assert golden["n_files"] > 50
     fixture_components = {"COMP_V", "COMP_W", "COMP_X", "COMP_Y", "COMP_Z"}
     # registered at run time by the reference's own tutorials / tests (add_custom_component) or by its inference entry point
     custom_or_runtime = {("inference_component", "text"), ("model", "einsum_transformer"), ("collate_fn", "custom_gpt_2_llm_collator"),
@@ -200,34 +192,18 @@ def test_component_nodes_of_the_reference_yaml_files_fit_our_schemas():
         ("model", "gpt2"): {"attention_norm", "ffn_norm", "lm_head_norm"},  # pre-``*_norm_config`` spelling in one tutorial file
     }
     problems, nodes = [], 0
-
-    def walk(node, where):
-        nonlocal nodes
-        if isinstance(node, dict):
-            if "component_key" in node and "variant_key" in node:
-                key = (node["component_key"], node["variant_key"])
-                if key[0] not in fixture_components and key not in custom_or_runtime and key not in stale_variants:
-                    nodes += 1
-                    entity = entities.get(key)
-                    if entity is None:
-                        problems.append((where, "unknown component", key))
-                    elif isinstance(node.get("config"), dict):
-                        schema = entity.component_config_type
-                        allowed = set(schema.model_fields) | set(getattr(schema, "__deprecated_aliases__", {}))
-                        extra = set(node["config"]) - allowed - known_stale.get(key, set())
-                        if extra:
-                            problems.append((where, key, sorted(extra)))
-            for k, v in node.items():
-                walk(v, f"{where}/{k}")
-        elif isinstance(node, list):
-            for i, v in enumerate(node):
-                walk(v, f"{where}[{i}]")
-
-    for f in files:
-        try:
-            content = yaml.safe_load(Path(f).read_text())
-        except yaml.YAMLError:
-            continue
-        walk(content, Path(f).relative_to(ref).as_posix())
+    for component, variant, config_keys, count, where in golden["nodes"]:
+        key = (component, variant)
+        if key[0] not in fixture_components and key not in custom_or_runtime and key not in stale_variants:
+            nodes += count
+            entity = entities.get(key)
+            if entity is None:
+                problems.append((where, "unknown component", key))
+            elif config_keys is not None:
+                schema = entity.component_config_type
+                allowed = set(schema.model_fields) | set(getattr(schema, "__deprecated_aliases__", {}))
+                extra = set(config_keys) - allowed - known_stale.get(key, set())
+                if extra:
+                    problems.append((where, key, sorted(extra)))
     assert nodes > 900
     assert not problems, problems[:20]

@@ -311,18 +311,15 @@ def test_cli_index_and_pack_with_shipped_config(tmp_path):
 
 
 def test_index_and_packed_file_are_byte_identical_to_the_reference_pipeline(tmp_path):
-    """The reference's own indexer + multi-process tokeniser / packer (baseline/_ref) and this framework's, driven through the
-    same library calls on the shipped corpus with the local GPT-2 tokenizer, write byte-identical ``.idx`` and ``.pbin``
-    files (md5)."""
-    import json
-    import subprocess
+    """The reference's own indexer + multi-process tokeniser / packer (the md5 of its files:
+    tests/golden/reference/data_pipeline.json.gz) and this framework's, driven through the same library calls on the shipped
+    corpus with the local GPT-2 tokenizer, write byte-identical ``.idx`` and ``.pbin`` files (md5)."""
     import sys
     from pathlib import Path
 
     repo = Path(__file__).resolve().parents[1]
-    if not (repo / "baseline" / "_ref" / "modalities").is_dir():
-        pytest.skip("the reference is not installed under baseline/_ref")
-    from conftest import run_arms
+    from conftest import reference_golden, run_arms
 
-    res = run_arms(lambda which: [sys.executable, "tests/workers/reference_data_pipeline.py", which, str(tmp_path / which)], cwd=repo)
+    res = run_arms(lambda which: [sys.executable, "tests/workers/reference_data_pipeline.py", which, str(tmp_path / which)], arms=("ours",), cwd=repo)
+    res["ref"] = reference_golden("data_pipeline")
     assert res["ours"] == res["ref"] and res["ref"]["pbin_bytes"] > 10_000, res

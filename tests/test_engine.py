@@ -248,7 +248,9 @@ def test_e2e_training_and_warmstart_across_world_sizes(tmp_path, lorem_pbin, fre
     checkpoints after steps 4 and 8, the checkpoint layout check, then a warm start from the step-4 checkpoint on ONE rank
     (DCP reshards) with twice the micro batch — the script itself asserts that steps 5-8 continue the uninterrupted curve
     (reference: tests/end2end_tests/test_fsdp2_warmstart_pp_tp.py, rel 1e-2). On top: the experiment-folder and checkpoint
-    artefacts of the first run, and the step-4 checkpoint loaded through the reference's own checkpoint classes."""
+    artefacts of the first run; the step-4 checkpoint holds every entry the reference's checkpoint classes write for this
+    model, with the same shape and dtype (tests/golden/reference/checkpoint_layout.json.gz), and loads into this
+    framework's plain single-process AppState."""
     env = dict(os.environ, MB200_DEVICE_TYPE="cpu", MB200_PARAM_DTYPE="FP_32", CUDA_VISIBLE_DEVICES="", MB200_DATA_PATH=str(lorem_pbin),
                MASTER_PORT=str(free_port))  # fmt: skip
     r = subprocess.run(["bash", "examples/warmstart/pre_train_and_warmstart.sh", str(tmp_path / "ws"), "2", "1", "gloo"], cwd=REPO, env=env,
@@ -266,54 +268,55 @@ def test_e2e_training_and_warmstart_across_world_sizes(tmp_path, lorem_pbin, fre
     assert sorted(p.name for p in (exp / "checkpoints" / ckpts[0]).iterdir()) == [".metadata", "__0_0.distcp", "__1_0.distcp"]
     assert info["checkpoint_folder_path"].endswith(ckpts[1])
     assert sorted(_losses(tmp_path / "ws" / "warmstart")) == [5, 6, 7, 8]
-    # the sharded checkpoint loads into the REFERENCE's own AppState + torch AdamW + OneCycleLR on a plain single process (DCP
-    # reshards) exactly like into this framework's: same weights, Adam moments and step, learning rate, scheduler position
-    if (REPO / "baseline" / "_ref" / "modalities").is_dir():
-        from conftest import run_arms
+    # what the REFERENCE's AppState + torch AdamW + OneCycleLR write for this model — and request when they load it — is the
+    # stored layout: the sharded checkpoint must hold each of those entries with the same shape and dtype. Then this
+    # framework's AppState loads it on a plain single process (DCP reshards) and restores Adam step and scheduler position.
+    from conftest import reference_golden
 
-        loaded = run_arms(lambda which: [sys.executable, "tests/workers/reference_checkpoint_load.py", which, str(exp / "checkpoints" / ckpts[0])],
-                          cwd=REPO)  # fmt: skip
-        assert loaded["ref"] == loaded["ours"], loaded
-        assert loaded["ref"]["adam_steps"] == [4.0] and loaded["ref"]["n_state"] == 21 and loaded["ref"]["sched_last_epoch"] == 4, loaded
+    def worker(*args):
+        r = subprocess.run([sys.executable, "tests/workers/reference_checkpoint_load.py", *args], cwd=REPO, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        return json.loads(r.stdout.strip().splitlines()[-1])
+
+    layout = worker("layout", str(exp / "checkpoints" / ckpts[0]))
+    wanted = reference_golden("checkpoint_layout")
+    assert {k: layout.get(k, "missing") for k in wanted} == wanted
+    loaded = worker("ours", str(exp / "checkpoints" / ckpts[0]))
+    assert loaded["adam_steps"] == [4.0] and loaded["n_state"] == 21 and loaded["sched_last_epoch"] == 4, loaded
 
 
 def test_pure_components_give_the_reference_implementations_results():
-    """tests/workers/reference_differential.py runs the same calls through the reference's own code (baseline/_ref) and through
-    this framework and the results must be EQUAL: the warm-up / cosine LR schedule (40 steps), the resumable sampler's index
-    sequences (shuffle / skip / drop_last / ranks), continuous packing over the shipped ``.pbin`` (lengths, first / last
-    samples, checksum), the next-token collator and the loss-masking wrapper, nine number-conversion functions, the CLM
+    """tests/workers/reference_differential.py runs the same calls through this framework as through the reference's own code
+    (its results: tests/golden/reference/differential.json.gz) and the results must be EQUAL: the warm-up / cosine LR
+    schedule (40 steps), the resumable sampler's index sequences (shuffle / skip / drop_last / ranks), continuous packing
+    over the shipped ``.pbin`` (lengths, first / last samples, checksum), the next-token collator and the loss-masking wrapper, nine number-conversion functions, the CLM
     cross entropy and both NCE variants, the composed and the Llama-3-like weight initialisation (per-parameter md5 of the
     bytes), seeded shuffles of tokenised / JSONL data and shuffled dataset chunks (file md5), combined and dummy datasets,
     the HF and SentencePiece tokenizer wrappers on the shipped tokenizer files, chunk ranges, and the sweep expansion of
     examples/scaling_up (sweep hash, per-world-size config hashes, md5 of every generated YAML), the checkpointing strategies'
     save / delete decisions, the DCP folder name, the ``evaluation_results.jsonl`` record and the MFU arithmetic."""
-    if not (REPO / "baseline" / "_ref" / "modalities").is_dir():
-        pytest.skip("the reference is not installed under baseline/_ref")
-    from conftest import run_arms
+    from conftest import reference_golden, run_arms
 
-    res = run_arms(lambda which: [sys.executable, "tests/workers/reference_differential.py", which], cwd=REPO)
+    res = run_arms(lambda which: [sys.executable, "tests/workers/reference_differential.py", which], arms=("ours",), cwd=REPO)
+    res["ref"] = reference_golden("differential")
     assert set(res["ref"]) == set(res["ours"]) and len(res["ref"]) >= 21
     for key, want in res["ref"].items():
         assert res["ours"][key] == want, key
     assert len(res["ref"]["weight_init"]) > 20 and len(res["ref"]["sampler"]) >= 13
 
 
-def test_models_are_numerically_identical_to_the_reference_implementation(tmp_path):
-    """Differential test against the reference's OWN model code (baseline/_ref): the reference builds a model, runs a
-    forward + backward on CPU and saves its state dict; this framework's model loads that state dict (strict: the FQNs and
-    shapes are the checkpoint contract) and must produce the same outputs, loss and parameter gradients — GPT2LLM with
+def test_models_are_numerically_identical_to_the_reference_implementation():
+    """Differential test against the reference's OWN model code: the reference built each model with weights seeded by
+    parameter name and recorded its state-dict layout, buffers, outputs, loss and parameter gradients on CPU
+    (tests/golden/reference/model_<variant>.json.gz); this framework's model must have the same layout (what a strict load
+    checks: the FQNs and shapes are the checkpoint contract) and produce the same outputs, loss and gradients — GPT2LLM with
     SwiGLU / GQA / RoPE / LayerNorm and with GELU / MHA / absolute positions / RMSNorm / biases / tied embeddings, CoCa (ViT
     encoder + attention pooling + text and multimodal decoders, 153 tensors) and the stand-alone ViT."""
-    if not (REPO / "baseline" / "_ref" / "modalities").is_dir():
-        pytest.skip("the reference is not installed under baseline/_ref")
+    from conftest import REFERENCE_GOLDEN
+
     variants = ["swiglu_gqa_rope_layernorm", "gelu_mha_abs_rmsnorm_bias_tied", "coca", "vit"]
-    procs = [subprocess.Popen([sys.executable, "tests/workers/reference_model_forward.py", "ref", str(tmp_path / f"{v}.pt"), v], cwd=REPO,
-                              stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True) for v in variants]  # fmt: skip
-    for v, p in zip(variants, procs):
-        _, err = p.communicate(timeout=600)
-        assert p.returncode == 0, (v, err[-3000:])
-    procs = [subprocess.Popen([sys.executable, "tests/workers/reference_model_forward.py", "ours", str(tmp_path / f"{v}.pt"), v], cwd=REPO,
-                              stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True) for v in variants]  # fmt: skip
+    procs = [subprocess.Popen([sys.executable, "tests/workers/reference_model_forward.py", "ours", str(REFERENCE_GOLDEN / f"model_{v}.json.gz"), v],
+                              cwd=REPO, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True) for v in variants]  # fmt: skip
     for v, p in zip(variants, procs):
         out, err = p.communicate(timeout=600)
         assert p.returncode == 0, (v, err[-3000:])
@@ -498,10 +501,9 @@ def test_reference_training_yaml_runs_unmodified_except_for_the_environment(name
     current settings schema requires it too (SURVEY §5.6 'stale settings.paths')."""
     import re
 
-    src = Path("/root/reference/config_files/training") / name
-    if not src.exists():
-        pytest.skip("reference checkout not available")
-    text = src.read_text()
+    from conftest import REFERENCE_GOLDEN
+
+    text = (REFERENCE_GOLDEN / name).read_text()
     fsdp1 = "fsdp1" in name  # the legacy surface has no device mesh and names its precision by preset
     patches = [
         ("    device_type: cuda", "    device_type: cpu", not fsdp1),

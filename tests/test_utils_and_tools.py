@@ -423,30 +423,14 @@ def test_reference_module_paths_resolve_through_the_alias_finder():
     import textwrap
     from pathlib import Path
 
-    ref_root = Path("/root/reference/src/modalities")
-    if ref_root.is_dir():
-        names = sorted(
-            ".".join(p.relative_to(ref_root).with_suffix("").parts).removesuffix(".__init__").removesuffix("__init__")
-            for p in ref_root.rglob("*.py")
-        )
-        names = [n for n in names if n and n != "__main__"]
-        # ... and every PUBLIC top-level name (classes, functions, upper-case constants) each of those modules defines
-        import ast
+    from conftest import reference_golden
 
-        public: dict[str, list[str]] = {}
-        for p in ref_root.rglob("*.py"):
-            mod = ".".join(p.relative_to(ref_root).with_suffix("").parts).removesuffix(".__init__").removesuffix("__init__")
-            if not mod or mod == "__main__" or mod == "conversion.gpt2.modeling_gpt2":
-                continue  # (modeling_gpt2: the exported HF model code; here an independent implementation with own helpers)
-            body = ast.parse(p.read_text()).body
-            defs = [n.name for n in body if isinstance(n, (ast.ClassDef, ast.FunctionDef)) and not n.name.startswith("_")]
-            defs += [t.id for n in body if isinstance(n, ast.Assign) for t in n.targets if isinstance(t, ast.Name) and t.id.isupper()]
-            public[mod] = defs
-        assert sum(map(len, public.values())) > 400
-    else:  # the recorded subset that differs from this package's layout
-        from modalities_b200.compat import MODULE_ALIASES
-
-        names, public = sorted(MODULE_ALIASES), {}
+    surface = reference_golden("surface")  # the reference's modules (tests/workers/reference_surface_probe.py extract)
+    names = sorted(surface)
+    # ... and every PUBLIC top-level name (classes, functions, upper-case constants) each of those modules defines
+    # (modeling_gpt2: the exported HF model code; here an independent implementation with own helpers)
+    public = {mod: s["defs"] for mod, s in surface.items() if mod != "conversion.gpt2.modeling_gpt2"}
+    assert len(names) > 100 and sum(map(len, public.values())) > 400
     code = textwrap.dedent(
         f"""
         import importlib, sys
@@ -553,7 +537,8 @@ def test_reference_names_for_user_code():
 def test_cli_command_tree_and_library_api_match_the_reference():
     """Every command of the reference's ``modalities`` CLI exists here with the same options (names, required, flags); the
     only additions are ``--backend`` on the distributed verbs. ``api.py``: same public functions / enums, same parameter
-    names and required-ness. Introspected from both packages (the reference from its installation under baseline/_ref)."""
+    names and required-ness. Introspected from this package and compared with the reference's introspection
+    (tests/golden/reference/cli_api.json.gz)."""
     import json
     import os
     import subprocess
@@ -561,12 +546,11 @@ def test_cli_command_tree_and_library_api_match_the_reference():
     from pathlib import Path
 
     repo = Path(__file__).resolve().parents[1]
-    if not (repo / "baseline" / "_ref" / "modalities").is_dir():
-        pytest.skip("the reference is not installed under baseline/_ref")
-    from conftest import run_arms
+    from conftest import reference_golden, run_arms
 
     env = dict(os.environ, PYTHONPATH=str(repo))
-    dumps = run_arms(lambda which: [sys.executable, str(repo / "tests" / "workers" / "cli_tree_dump.py"), which], cwd=repo, env=env)
+    dumps = run_arms(lambda which: [sys.executable, str(repo / "tests" / "workers" / "cli_tree_dump.py"), which], arms=("ours",), cwd=repo, env=env)
+    dumps["ref"] = reference_golden("cli_api")
     assert dumps["ours"]["api"] == dumps["ref"]["api"] and len(dumps["ref"]["api"]) >= 12, (dumps["ours"]["api"], dumps["ref"]["api"])
     ours, ref = dumps["ours"]["cli"], dumps["ref"]["cli"]
     assert set(ours) == set(ref) and len(ref) >= 15, (sorted(set(ref) - set(ours)), sorted(set(ours) - set(ref)))
@@ -586,8 +570,6 @@ def test_public_classes_methods_and_parameter_names_match_the_reference():
     import sys
     from pathlib import Path
 
-    if not Path("/root/reference/src/modalities").is_dir():
-        pytest.skip("needs the reference checkout")
     repo = Path(__file__).resolve().parents[1]
     r = subprocess.run([sys.executable, str(repo / "tests" / "workers" / "reference_surface_probe.py")], capture_output=True, text=True, cwd=repo)
     assert r.returncode == 0, r.stderr[-3000:]
@@ -606,11 +588,10 @@ def test_every_pydantic_schema_and_enum_of_the_reference_has_the_same_fields_her
     from pathlib import Path
 
     repo = Path(__file__).resolve().parents[1]
-    if not (repo / "baseline" / "_ref" / "modalities").is_dir():
-        pytest.skip("the reference is not installed under baseline/_ref")
-    from conftest import run_arms
+    from conftest import reference_golden, run_arms
 
-    dumps = run_arms(lambda which: [sys.executable, str(repo / "tests" / "workers" / "pydantic_schema_dump.py"), which], cwd=repo)
+    dumps = run_arms(lambda which: [sys.executable, str(repo / "tests" / "workers" / "pydantic_schema_dump.py"), which], arms=("ours",), cwd=repo)
+    dumps["ref"] = reference_golden("pydantic_schemas")
     # enums (37): same members, same values where the value is a literal (MixedPrecisionSettings maps onto other policy objects)
     for name, members in dumps["ref"]["enums"].items():
         mine = dumps["ours"]["enums"].get(name)

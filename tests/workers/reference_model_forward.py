@@ -1,9 +1,14 @@
-"""Builds a tiny GPT2LLM with the REFERENCE implementation (baseline/_ref), runs forward + backward on CPU in fp32 and
-saves the state dict, inputs, logits and gradients — or, with ``ours``, loads that file into THIS framework's GPT2LLM (the
-FQNs are the contract) and reports the differences. Usage: reference_model_forward.py {ref|ours} <file.pt> <variant>"""
+"""Builds a tiny model (GPT2LLM variants, CoCa, ViT) with the REFERENCE implementation (``ref``: baseline/_ref) or with THIS
+framework (``ours``), sets every parameter from a generator seeded by its name (the FQNs are the checkpoint contract),
+runs forward + backward on CPU in fp32. ``ref`` writes the state-dict layout and a record of its outputs, loss and
+gradients (exact values at fixed, seeded positions plus sum and norm of every tensor) to <file.json.gz>; ``ours`` reads
+that record and reports the differences. Usage: reference_model_forward.py {ref|ours} <file.json.gz> <variant>"""
 
+import gzip
 import json
+import math
 import sys
+import zlib
 from pathlib import Path
 
 import torch
@@ -11,17 +16,87 @@ import torch
 REPO = Path(__file__).resolve().parents[2]
 sys.path.insert(0, str(REPO))
 which, path, variant = sys.argv[1], sys.argv[2], sys.argv[3]
-if variant in ("coca", "vit"):
+N_SAMPLES = 4  # recorded elements per gradient tensor (model outputs: 128)
+
+
+def seeded_init(model):
+    """Every floating parameter from a generator seeded by its state-dict name: matrices ~ N(0, 0.05), vectors 1 + N(0, 0.05)
+    (weights: norm scales) or N(0, 0.05) (biases). Tied tensors take the value of their last name in sorted order."""
+    with torch.no_grad():
+        for name, t in sorted(model.state_dict(keep_vars=True).items()):
+            if not isinstance(t, torch.nn.Parameter) or not t.is_floating_point():
+                continue
+            noise = 0.05 * torch.randn(t.shape, generator=torch.Generator().manual_seed(zlib.crc32(name.encode())))
+            t.copy_(noise if t.dim() > 1 else noise + (1.0 if name.endswith("weight") else 0.0))
+
+
+def positions(n, n_samples):
+    return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:n_samples].sort().values
+
+
+def record(t, n_samples):
+    flat = t.detach().double().reshape(-1)
+    return {"shape": list(t.shape), "sum": float(f"{flat.sum().item():.12g}"), "sumsq": float(f"{flat.square().sum().item():.12g}"),
+            "val": [float(f"{v:.9g}") for v in flat[positions(flat.numel(), n_samples)].tolist()]}  # fmt: skip
+
+
+def deviation(t, rec):
+    """A lower bound of max |t - recorded tensor|: at the recorded positions, of the means and of the norms."""
+    assert list(t.shape) == rec["shape"], (list(t.shape), rec["shape"])
+    flat = t.detach().double().reshape(-1)
+    n = flat.numel()
+    at = (flat[positions(n, len(rec["val"]))] - torch.tensor(rec["val"], dtype=torch.float64)).abs().max().item()
+    return max(at, abs(flat.sum().item() - rec["sum"]) / n, abs(flat.square().sum().item() ** 0.5 - rec["sumsq"] ** 0.5) / math.sqrt(n))
+
+
+def layout(model):
+    sd = model.state_dict()
+    buffers = {n for n, _ in model.named_buffers()}
+    return {n: list(t.shape) for n, t in sd.items()}, {n: t for n, t in sd.items() if n in buffers}
+
+
+def finish(model, outputs: dict, loss):
+    grads = {n: p.grad for n, p in model.named_parameters() if p.grad is not None}
+    state, buffers = layout(model)
     if which == "ref":
-        sys.path.insert(0, str(REPO / "baseline"))
-        import ref_env
+        Path(path).write_bytes(gzip.compress(json.dumps({
+            "state": state, "buffers": {n: record(b, N_SAMPLES) for n, b in buffers.items()}, "loss": None if loss is None else loss.item(),
+            "out": {k: record(v, 128) for k, v in outputs.items()}, "grads": {n: record(g, N_SAMPLES) for n, g in grads.items()},
+        }).encode(), mtime=0))  # fmt: skip
+        print(json.dumps({"saved": True, "n_params": sum(p.numel() for p in model.parameters())}))
+        return
+    assert set(grads) == set(blob["grads"]), sorted(set(grads) ^ set(blob["grads"]))
+    print(json.dumps({
+        "logit_diff": max(deviation(v, blob["out"][k]) for k, v in outputs.items()),
+        "loss_diff": 0.0 if loss is None else abs(loss.item() - blob["loss"]),
+        "grad_diff": max(deviation(grads[n], rec) for n, rec in blob["grads"].items()), "n_tensors": len(state),
+    }))  # fmt: skip
 
-        ref_env.prepare()
-    else:
-        import modalities_b200  # noqa: F401
-        from modalities_b200 import compat
 
-        compat.install_modalities_alias()
+def prepare(model):
+    """ours: the state-dict layout (what a strict load of the reference's checkpoint checks) and the buffers in it must be
+    the reference's."""
+    seeded_init(model)
+    if which == "ours":
+        state, buffers = layout(model)
+        assert state == blob["state"], sorted(k for k in set(state) | set(blob["state"]) if state.get(k) != blob["state"].get(k))[:10]
+        for n, rec in blob["buffers"].items():
+            assert deviation(buffers[n].float(), rec) < 1e-6, n
+    return model
+
+
+if which == "ref":
+    sys.path.insert(0, str(REPO / "baseline"))
+    import ref_env
+
+    ref_env.prepare()
+else:
+    import modalities_b200  # noqa: F401
+    from modalities_b200 import compat
+
+    compat.install_modalities_alias()
+    blob = json.loads(gzip.decompress(Path(path).read_bytes()))
+if variant in ("coca", "vit"):
     torch.manual_seed(0)
     if variant == "coca":
         from modalities.models.coca.coca_model import CoCa, CoCaConfig
@@ -49,26 +124,10 @@ if variant in ("coca", "vit"):
         keys = ["logits"]
     g = torch.Generator().manual_seed(1)
     batch = {"images": torch.randn(3, 3, 32, 32, generator=g), "input_ids": torch.randint(0, 97, (3, 16), generator=g)}
-    if which == "ref":
-        with torch.no_grad():
-            for p in model.parameters():
-                torch.nn.init.normal_(p, 0.0, 0.05) if p.dim() > 1 else p.add_(0.05 * torch.randn_like(p))
-        out = model(batch)
-        sum(out[k].float().pow(2).mean() for k in keys).backward()
-        torch.save({"state": model.state_dict(), "out": {k: out[k].detach() for k in keys},
-                    "grads": {n: p.grad for n, p in model.named_parameters() if p.grad is not None}}, path)  # fmt: skip
-        print(json.dumps({"saved": True}))
-    else:
-        blob = torch.load(path, weights_only=False)
-        model.load_state_dict(blob["state"], strict=True)
-        out = model(batch)
-        sum(out[k].float().pow(2).mean() for k in keys).backward()
-        grads = {n: p.grad for n, p in model.named_parameters() if p.grad is not None}
-        assert set(grads) == set(blob["grads"]), sorted(set(grads) ^ set(blob["grads"]))
-        print(json.dumps({
-            "logit_diff": max((out[k] - blob["out"][k]).abs().max().item() for k in keys), "loss_diff": 0.0,
-            "grad_diff": max((grads[n] - gr).abs().max().item() for n, gr in blob["grads"].items()), "n_tensors": len(blob["state"]),
-        }))  # fmt: skip
+    model = prepare(model)
+    out = model(batch)
+    sum(out[k].float().pow(2).mean() for k in keys).backward()
+    finish(model, {k: out[k] for k in keys}, None)
     sys.exit(0)
 d = 128
 norm_type, act, n_kv, poe, bias, tie = {
@@ -83,39 +142,13 @@ cfg = dict(
     attention_config={"qkv_transforms": rope if poe == "NOPE" else []}, attention_implementation="pytorch_flash",
     activation_type=act, attention_norm_config=norm, ffn_norm_config=norm, lm_head_norm_config=norm, use_weight_tying=tie,
 )  # fmt: skip
-if which == "ref":
-    sys.path.insert(0, str(REPO / "baseline"))
-    import ref_env
+from modalities.models.gpt2.gpt2_model import GPT2LLM, GPT2LLMConfig  # noqa: E402
 
-    ref_env.prepare()
-    from modalities.models.gpt2.gpt2_model import GPT2LLM, GPT2LLMConfig
-else:
-    from modalities_b200.models.gpt2.gpt2_model import GPT2LLM, GPT2LLMConfig
 c = GPT2LLMConfig(**cfg)
 torch.manual_seed(0)
-model = GPT2LLM(**{k: getattr(c, k) for k in type(c).model_fields if k != "use_meta_device"}).float()
-if which == "ref":
-    with torch.no_grad():
-        for p in model.parameters():
-            torch.nn.init.normal_(p, 0.0, 0.05) if p.dim() > 1 else p.add_(0.05 * torch.randn_like(p))
-    ids = torch.randint(0, 256, (2, 65), generator=torch.Generator().manual_seed(1))
-    logits = model({"input_ids": ids[:, :-1]})["logits"]
-    loss = torch.nn.functional.cross_entropy(logits.reshape(-1, 256), ids[:, 1:].reshape(-1))
-    loss.backward()
-    torch.save({"state": model.state_dict(), "ids": ids, "logits": logits.detach(), "loss": loss.item(),
-                "grads": {n: p.grad for n, p in model.named_parameters()}}, path)  # fmt: skip
-    print(json.dumps({"saved": True, "n_params": sum(p.numel() for p in model.parameters())}))
-else:
-    blob = torch.load(path, weights_only=False)
-    missing, unexpected = model.load_state_dict(blob["state"], strict=True), None
-    ids = blob["ids"]
-    logits = model({"input_ids": ids[:, :-1]})["logits"]
-    loss = torch.nn.functional.cross_entropy(logits.reshape(-1, 256), ids[:, 1:].reshape(-1))
-    loss.backward()
-    grads = {n: p.grad for n, p in model.named_parameters()}
-    assert set(grads) == set(blob["grads"]), (sorted(set(grads) ^ set(blob["grads"])))
-    print(json.dumps({
-        "logit_diff": (logits - blob["logits"]).abs().max().item(), "loss_diff": abs(loss.item() - blob["loss"]),
-        "grad_diff": max((grads[n] - g).abs().max().item() for n, g in blob["grads"].items()),
-        "n_tensors": len(blob["state"]),
-    }))  # fmt: skip
+model = prepare(GPT2LLM(**{k: getattr(c, k) for k in type(c).model_fields if k != "use_meta_device"}).float())
+ids = torch.randint(0, 256, (2, 65), generator=torch.Generator().manual_seed(1))
+logits = model({"input_ids": ids[:, :-1]})["logits"]
+loss = torch.nn.functional.cross_entropy(logits.reshape(-1, 256), ids[:, 1:].reshape(-1))
+loss.backward()
+finish(model, {"logits": logits}, loss)

@@ -1,11 +1,15 @@
 """Compares the public surface of every reference module with what its import path resolves to here (through the alias
 finder): public methods / annotated fields of every public class, and the parameter NAMES of every public function,
-method and constructor. Prints a JSON report; tests/test_utils_and_tools.py asserts that it is empty.
+method and constructor. The reference's surface is read from tests/golden/reference/surface.json.gz (written by
+``extract`` from a reference checkout, see scripts/reference_goldens.py). Prints a JSON report;
+tests/test_utils_and_tools.py asserts that it is empty.
 
-    python tests/workers/reference_surface_probe.py [/root/reference/src/modalities]
+    python tests/workers/reference_surface_probe.py                          # check this package
+    python tests/workers/reference_surface_probe.py extract <src/modalities>  # print the surface of a reference checkout
 """
 
 import ast
+import gzip
 import importlib
 import inspect
 import json
@@ -13,19 +17,47 @@ import os
 import sys
 from pathlib import Path
 
-sys.path.insert(0, str(Path(__file__).resolve().parents[2]))
-import modalities_b200  # noqa: E402,F401
-from modalities_b200 import compat  # noqa: E402
-
-compat.install_modalities_alias()
-root = sys.argv[1] if len(sys.argv) > 1 else "/root/reference/src/modalities"
+REPO = Path(__file__).resolve().parents[2]
+GOLDEN = REPO / "tests" / "golden" / "reference" / "surface.json.gz"
 SKIP = {"__main__", "conversion.gpt2.modeling_gpt2"}  # (the exported HF model code is an independent implementation here)
-report = {"missing_members": {}, "missing_parameters": {}, "classes": 0, "methods": 0, "callables": 0}
 
 
 def ref_params(fn):
     a = fn.args
     return [x.arg for x in a.posonlyargs + a.args + a.kwonlyargs if x.arg not in ("self", "cls")]
+
+
+def extract(root: str) -> dict:
+    """{module: {"defs": public top-level names, "functions": {name: params},
+    "classes": {name: {"methods": [...], "fields": [...], "callables": {method: params}}}}} of every module under root."""
+    surface = {}
+    for dp, _, fs in os.walk(root):
+        for f in sorted(fs):
+            if not f.endswith(".py"):
+                continue
+            rel = os.path.relpath(os.path.join(dp, f), root)[:-3].replace(os.sep, ".")
+            rel = rel.removesuffix(".__init__").removesuffix("__init__")
+            if not rel or rel == "__main__":
+                continue
+            body = ast.parse(open(os.path.join(dp, f)).read()).body
+            defs = [n.name for n in body if isinstance(n, (ast.ClassDef, ast.FunctionDef)) and not n.name.startswith("_")]
+            defs += [t.id for n in body if isinstance(n, ast.Assign) for t in n.targets if isinstance(t, ast.Name) and t.id.isupper()]
+            functions, classes = {}, {}
+            for node in body:
+                if isinstance(node, ast.FunctionDef) and not node.name.startswith("_"):
+                    functions[node.name] = ref_params(node)
+                if isinstance(node, ast.ClassDef) and not node.name.startswith("_"):
+                    c = classes[node.name] = {"methods": [], "fields": [], "callables": {}}
+                    for b in node.body:
+                        if isinstance(b, (ast.FunctionDef, ast.AsyncFunctionDef)):
+                            if not b.name.startswith("_"):
+                                c["methods"].append(b.name)
+                            if not b.name.startswith("_") or b.name == "__init__":
+                                c["callables"][b.name] = ref_params(b)
+                        elif isinstance(b, ast.AnnAssign) and isinstance(b.target, ast.Name) and not b.target.id.startswith("_"):
+                            c["fields"].append(b.target.id)
+            surface[rel] = {"defs": defs, "functions": functions, "classes": classes}
+    return dict(sorted(surface.items()))
 
 
 def our_params(obj):
@@ -37,46 +69,45 @@ def our_params(obj):
     return names, any(p.kind == p.VAR_KEYWORD for p in sig.parameters.values())
 
 
-for dp, _, fs in os.walk(root):
-    for f in fs:
-        if not f.endswith(".py"):
+def check(surface: dict) -> dict:
+    sys.path.insert(0, str(REPO))
+    import modalities_b200  # noqa: F401
+    from modalities_b200 import compat
+
+    compat.install_modalities_alias()
+    report = {"missing_members": {}, "missing_parameters": {}, "classes": 0, "methods": 0, "callables": 0}
+    for rel, mod in surface.items():
+        if rel in SKIP:
             continue
-        rel = os.path.relpath(os.path.join(dp, f), root)[:-3].replace(os.sep, ".")
-        rel = rel.removesuffix(".__init__").removesuffix("__init__")
-        if not rel or rel in SKIP:
-            continue
-        tree = ast.parse(open(os.path.join(dp, f)).read())
         m = importlib.import_module("modalities." + rel)
-        callables = []
-        for node in tree.body:
-            if isinstance(node, ast.FunctionDef) and not node.name.startswith("_") and hasattr(m, node.name):
-                callables.append((node.name, node, getattr(m, node.name)))
-            if isinstance(node, ast.ClassDef) and not node.name.startswith("_") and hasattr(m, node.name):
-                cls = getattr(m, node.name)
-                report["classes"] += 1
-                fields = set(getattr(cls, "model_fields", None) or {}) | set(getattr(cls, "__dataclass_fields__", None) or {})
-                fields |= set(getattr(cls, "__annotations__", None) or {})
-                missing = []
-                for b in node.body:
-                    if isinstance(b, (ast.FunctionDef, ast.AsyncFunctionDef)):
-                        if not b.name.startswith("_"):
-                            report["methods"] += 1
-                            if not hasattr(cls, b.name):
-                                missing.append(b.name)
-                        if (not b.name.startswith("_") or b.name == "__init__") and hasattr(cls, b.name):
-                            callables.append((f"{node.name}.{b.name}", b, getattr(cls, b.name)))
-                    elif isinstance(b, ast.AnnAssign) and isinstance(b.target, ast.Name) and not b.target.id.startswith("_"):
-                        if not hasattr(cls, b.target.id) and b.target.id not in fields:
-                            missing.append(b.target.id)
-                if missing:
-                    report["missing_members"][f"{rel}.{node.name}"] = missing
-        for name, node, obj in callables:
+        callables = [(name, params, getattr(m, name)) for name, params in mod["functions"].items() if hasattr(m, name)]
+        for cname, c in mod["classes"].items():
+            if not hasattr(m, cname):
+                continue
+            cls = getattr(m, cname)
+            report["classes"] += 1
+            fields = set(getattr(cls, "model_fields", None) or {}) | set(getattr(cls, "__dataclass_fields__", None) or {})
+            fields |= set(getattr(cls, "__annotations__", None) or {})
+            report["methods"] += len(c["methods"])
+            missing = [b for b in c["methods"] if not hasattr(cls, b)]
+            missing += [b for b in c["fields"] if not hasattr(cls, b) and b not in fields]
+            callables += [(f"{cname}.{b}", params, getattr(cls, b)) for b, params in c["callables"].items() if hasattr(cls, b)]
+            if missing:
+                report["missing_members"][f"{rel}.{cname}"] = missing
+        for name, params, obj in callables:
             ours = our_params(obj)
             if ours is None:
                 continue
             report["callables"] += 1
             names, has_kwargs = ours
-            lacking = [p for p in ref_params(node) if p not in names]
+            lacking = [p for p in params if p not in names]
             if lacking and not has_kwargs:
                 report["missing_parameters"][f"{rel}.{name}"] = lacking
-print(json.dumps(report))
+    return report
+
+
+if __name__ == "__main__":
+    if len(sys.argv) > 2 and sys.argv[1] == "extract":
+        print(json.dumps(extract(sys.argv[2])))
+    else:
+        print(json.dumps(check(json.loads(gzip.decompress(GOLDEN.read_bytes())))))
